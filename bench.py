@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference's CPU path (oracle port), rank 0 only
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N    # one process per GPU, NCCL gradient all-reduce
+    python bench.py ... --dump-outputs DIR      # also write what the last timed step computed to DIR/*.npy (rank 0)
 
 Workload = BASELINE config 2 ("Atari Pong DQN, 1M-transition PrioritizedExperienceReplay, 84x84x4 uint8, batch 512"):
 per GPU one HBM-resident replay shard with a 2^20-leaf fp64 sum/min/max tree and 2^20 ring slots (59.2 GB), synthetic
@@ -207,6 +208,33 @@ def build_device_agent(capacity, seed, device, config="dqn", frame_dedup=False):
     return agent
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(agent, out_dir):
+    """Writes what the last learn step computed, as a caller of Agent.train() / learn_from_batch sees it, to
+    out_dir/<name>.npy: the loss and the squared global gradient norm the step returns, its sampled batch (leaf
+    indices, importance weights), TD targets and errors, the priorities written back to the sampled leaves of the sum
+    tree, and the online network's parameters after the optimizer step.  float32 / float64 only (the leaf indices are
+    exact in float64).  The inputs depend only on the command-line arguments, so two builds can be compared file by
+    file."""
+    import torch
+    torch.cuda.synchronize()
+    net, mem, bb = agent.networks["main"], agent.memory, agent.batch_buffers
+    idx = bb["idx"]
+    outs = {"loss": agent.loss_dev, "grad_sumsq": net.sumsq, "idx": idx.to(torch.float64),
+            "is_weights": bb["weight"], "td_targets": agent.targets, "td_errors": agent.td_err,
+            "priorities": mem.sum_tree[mem.power_of_2_size - 1 + idx], "online_params": net.store.theta}
+    outs = {k: v.detach().cpu().numpy() for k, v in outs.items()}
+    for k, v in outs.items():
+        assert v.dtype in (np.float32, np.float64), (k, v.dtype)
+    total = sum(v.nbytes for v in outs.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs of one step: %d bytes" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in outs.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def host_transitions(rng, n, stacked_by_filter=False):
     """n new host-side transitions (what Agent.observe would hand to memory.store).  stacked_by_filter: the states are
     the LazyStacks an ObservationStackingFilter(4) hands out along one episode (one new 84x84 frame per transition,
@@ -295,6 +323,8 @@ def run_device(args):
         agent._join_optimizer()            # the last step's optimizer part (own stream) belongs to the timed region
     t1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(agent, args.dump_outputs)        # before any untimed step below changes the agent's state
     agent.sample_batch = orig_sample
     mem.kernel_events = None
     ms_total = t0.elapsed_time(t1)
@@ -565,7 +595,6 @@ def run_reference(args):
     if rank != 0:
         return
     K, W = args.steps, args.warmup
-    K = min(K, 40)                      # bounded: the CPU step takes a sizeable fraction of a second
     W = max(3, min(W, 10))              # same warm-up as the device arm (bounded: a CPU step is ~0.2 s)
     base = cpu_reference(steps=K, warmup=W)
     line = {"impl": "reference", "metric": "learn_from_batch steps/sec (DQN PER batch 512)", "value": base["value"],
@@ -620,7 +649,14 @@ def main():
                     help="dqn: BASELINE config 2 (Atari DQN + PER, the headline metric, default); dueling: config 5 "
                          "(dueling DDQN + PER, no middleware, clip-norm 10); cartpole / ppo / sac / td3: configs 1, 3, 4 "
                          "(bench_configs.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, sampled batch, TD errors, priorities, network "
+                         "parameters) to DIR/<name>.npy; dqn / dueling configurations of this repo's CUDA path")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config not in ("dqn", "dueling")):
+        ap.error("--dump-outputs covers the dqn and dueling configurations of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     elif args.config in ("cartpole", "ppo", "sac", "td3"):

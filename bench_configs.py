@@ -199,7 +199,7 @@ def _ppo(args, torch, parallel, lib, device, rank, world, local, K, W, barrier, 
     done = (rng.rand(n) < 1.0 / 500).astype(np.uint8)
     done[T - 1::T] = 1                                                     # forced at the end of every env's rollout
     cols["game_over"] = done
-    K, W = min(K, 5), min(W, 2)                # a phase is 20,480 minibatch steps: seconds, not milliseconds
+    W = min(W, 2)                              # a phase is 20,480 minibatch steps: seconds, not milliseconds
     phase_ms = []
 
     def step():

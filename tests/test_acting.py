@@ -1,42 +1,28 @@
 """The batched epsilon-greedy of the device acting path against the UNMODIFIED reference policy objects (one EGreedy per
-environment, all drawing from numpy's global generator in agent order).  CPU only; skipped without /root/reference."""
+environment, all drawing from numpy's global generator in agent order).  CPU only.  The reference's actions are stored
+in tests/golden/e_greedy.npz (oracle/make_golden_boundary.py)."""
+import os
+
 import numpy as np
 import pytest
 
-from oracle import ref_loader
 
-needs_ref = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-
-
-@needs_ref
 @pytest.mark.parametrize("test_phase", [False, True])
-def test_batched_e_greedy_selects_the_reference_actions(test_phase):
-    ref_loader.load()
-    from rl_coach.core_types import RunPhase as RefPhase
-    from rl_coach.exploration_policies.e_greedy import EGreedy
-    from rl_coach.schedules import LinearSchedule as RefLinear
-    from rl_coach.spaces import DiscreteActionSpace
+def test_batched_e_greedy_selects_the_reference_actions(test_phase, golden_dir):
     from coach_b200.exploration_policies.e_greedy import BatchedEGreedy, RunPhase
     from coach_b200.schedules import LinearSchedule
-    E, A, T = 5, 6, 40
-    rng = np.random.RandomState(0)
-    q = rng.randn(T, E, A).astype(np.float32)
-    q[3, 1, 2] = q[3, 1, 4] = q[3, 1].max() + 1.0            # exact ties: random tie-break consumes the stream
-    q[7, 0] = 0.5
-    np.random.seed(11)
-    refs = [EGreedy(DiscreteActionSpace(A), RefLinear(1.0, 0.1, 25), 0.05) for _ in range(E)]
-    for p in refs:
-        p.change_phase(RefPhase.TEST if test_phase else RefPhase.TRAIN)
-    want = np.zeros((T, E), dtype=np.int64)
-    for t in range(T):
-        for e in range(E):
-            want[t, e], _ = refs[e].get_action(q[t, e])
-    np.random.seed(11)
-    mine = BatchedEGreedy(A, E, LinearSchedule(1.0, 0.1, 25), 0.05)
+    fx = np.load(os.path.join(golden_dir, "e_greedy.npz"))
+    q = fx["q"]
+    T, E, A = q.shape
+    tag = "test" if test_phase else "train"
+    want = fx["actions_" + tag]
+    np.random.seed(int(fx["seed"]))
+    mine = BatchedEGreedy(A, E, LinearSchedule(float(fx["start"]), float(fx["end"]), int(fx["decay_steps"])),
+                          float(fx["evaluation_epsilon"]))
     mine.change_phase(RunPhase.TEST if test_phase else RunPhase.TRAIN)
     got = np.zeros((T, E), dtype=np.int64)
     for t in range(T):
         got[t], probs = mine.get_actions(q[t])
         assert np.allclose(probs.sum(1), 1.0)
     np.testing.assert_array_equal(got, want)
-    assert float(mine.epsilon_schedules[0].current_value) == float(refs[0].epsilon_schedule.current_value)
+    assert float(mine.epsilon_schedules[0].current_value) == float(fx["epsilon_" + tag])
